@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — denoising steps/sec of the MagCache hot path on Wan2.1-T2V-1.3B, 832x480x81 frames (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-cache]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-cache] [--dump-outputs DIR]
 
 One "step" = one denoising step = the cond + uncond pair of patched-forward calls the reference's caller makes
 (eval/magcache/experiments/Wan2.1_EVAL/wan_magcache.py:296-299) under the E012K4R02 schedule
@@ -54,6 +54,21 @@ def select_workload(name):
         ATTN_SELF_FLOPS = 4.0 * N_TOK * N_TOK * D
         FWD_FLOPS = 6523.0e12  # SURVEY §8d
         WORKLOAD, MODEL_KEY, TABLE = "Wan2.1-T2V-14B 1280x720x81f", "t2v-14B", "wan2.1_t2v_14b"
+
+
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the arrays the timed path returned in its last step, as <out_dir>/<name>.npy in float32. The inputs and
+    weights are seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    host = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_BYTES_MAX, f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES_MAX}-byte budget"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -198,13 +213,10 @@ def run_reference_arm(args, rank):
     if args.warmup > 0:
         cpu_cycle(state)
     tm, th = [], []
-    t_start = time.perf_counter()
-    for _ in range(max(1, args.steps)):
+    for _ in range(args.steps):
         a, b = cpu_cycle(state)
         tm.append(a)
         th.append(b)
-        if time.perf_counter() - t_start > 120:  # keep the whole run within a few minutes
-            break
     t_miss_small, t_hit = statistics.median(tm), statistics.median(th)
     value, sec_video, t_miss = cpu_extrapolate(t_miss_small, t_hit)
     sample = cpu_sample_text(len(tm), cores, t_miss_small, t_hit, t_miss, sec_video)
@@ -335,6 +347,8 @@ def run_ours(args, rank, world):
     live_tags = {"attn_self", "head", "head_hit_fused"}  # recorded live inside the timed region; the full attribution runs separately
     ms, launches, clocks, prof, x_final, per_fwd = timed(step_resident, args.steps, False if graphs else live_tags, args.warmup)
     assert torch.isfinite(x_final).all(), "non-finite latents after the timed steps"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"latent": x_final})
     ms_e2e, _, _, _, _, _ = timed(step_e2e, args.steps, False, args.warmup)
     roofline_source = "CUDA events around every launch inside the timed region"
 
@@ -577,7 +591,7 @@ def run_mmdit(args, rank, world):
                 o = call(i, x, c)
                 out_h.view(-1)[:o.numel()].copy_(o.reshape(-1), non_blocking=True)
             else:
-                call(i, hs, enc)
+                o = call(i, hs, enc)
         e1.record()
         barrier()
         clocks = sampler.stop()
@@ -587,10 +601,12 @@ def run_mmdit(args, rank, world):
             tms = torch.tensor([t_ms], device=dev)
             dist.all_reduce(tms, op=dist.ReduceOp.MAX)
             t_ms = float(tms.item())
-        return t_ms, ops.LAUNCHES - n0, clocks, prof
+        return t_ms, ops.LAUNCHES - n0, clocks, prof, o
 
-    ms, launches, clocks, prof = timed(False, {"mmdit_attn"})
-    ms_e2e, _, _, _ = timed(True, None)
+    ms, launches, clocks, prof, out = timed(False, {"mmdit_attn"})
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"prediction": out})
+    ms_e2e, _, _, _, _ = timed(True, None)
     pk = peaks()
     S = n_img + n_txt
     attn_flops = 4.0 * (n_img // world + n_txt) * S * heads * 128  # per GPU: its image rows + the replicated text rows x all keys
@@ -707,10 +723,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cache", action="store_true", help="time the non-cached DiT loop at identical shapes")
     ap.add_argument("--skip-cpu", action="store_true", help="omit the cpu_baseline leg (debugging)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32)")
     ap.add_argument("--workload", default="wan1.3b", choices=["wan1.3b", "wan14b", "flux", "hunyuan720p"],
                     help="wan14b: BASELINE configs[4] model/shape; flux: configs[0] (FLUX.1-dev 1024x1024, 28 steps); hunyuan720p: configs[3] "
                          "(720p x 129 frames, 50 steps) — none of these is the driver's metric")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm's timed cycle keeps no outputs")
     select_workload(args.workload)
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
