@@ -9,9 +9,10 @@ the forwards' own statements (embedders, controller, hit / miss, residual, final
 (`MMDiTCore`): same modulation chunk order, same per-head q/k RMSNorm, same `cat(attn, act(mlp))` single block; they differ in the
 token order of the joint sequence, in which rows get RoPE, and in their embedders.
 
-STATUS (end of round 1): parity-green on a B200 against the oracles at reduced depth / token counts (tests/test_flux_forward_gpu.py,
-tests/test_hunyuan_forward_gpu.py; profiles/r01_mmdit_first_gpu_run.md) and pinned on CPU through the kernel emulation
-(tests/test_*_engine_emulated_cpu.py); not yet run or timed at the full FLUX 1024^2 / HunyuanVideo 720p shapes. Nothing on the Wan path
+STATUS: parity-green on a B200 against the oracles at reduced depth / token counts (tests/test_flux_forward_gpu.py,
+tests/test_hunyuan_forward_gpu.py) and pinned on CPU through the kernel emulation (tests/test_*_engine_emulated_cpu.py); run and timed at
+full size with synthetic weights by `bench.py --workload flux|hunyuan720p` (profiles/r02_bench_flux_1024.json,
+profiles/r02_bench_hunyuan_720p.json, and token-sharded over 2 GPUs profiles/r02_bench_hunyuan_720p_2gpu.json). Nothing on the Wan path
 depends on this module.
 
 HBM layout (S = n_txt + n_img tokens; FLUX puts the text rows FIRST — `torch.cat([encoder_hidden_states, hidden_states], dim=1)`,
@@ -28,16 +29,32 @@ import numpy as np
 import torch
 
 from . import _lib, ops
+from .wan import _bf16, _bias_autocast
 
 E = _lib
 
 
-def _w(t, dev):
-    return t.detach().to(device=dev, dtype=torch.bfloat16).contiguous()
+def _mlp2(lin1, lin2, dev):
+    """(w1, b1, w2, b2) of a two-Linear embedder MLP."""
+    return _bf16(lin1.weight, dev), _bias_autocast(lin1.bias, dev), _bf16(lin2.weight, dev), _bias_autocast(lin2.bias, dev)
 
 
-def _b(t, dev):
-    return t.detach().to(device=dev, dtype=torch.bfloat16).float().contiguous()  # bf16 parameter values, kept as fp32 for the epilogues
+class _AdaStack:
+    """The Linear projections of a forward's AdaLayerNorm / ModulateDiT layers stacked into one matrix (they all read the same
+    conditioning vector: one GEMM computes them). `add` returns a projection's first row in the stack."""
+
+    def __init__(self):
+        self.ws, self.bs, self.rows = [], [], 0
+
+    def add(self, lin):
+        self.ws.append(lin.weight.detach())
+        self.bs.append(lin.bias.detach())
+        start, self.rows = self.rows, self.rows + lin.weight.shape[0]
+        return start
+
+    def pack(self, dev):
+        """(weight bf16, bias fp32, rows) of the stack."""
+        return _bf16(torch.cat(self.ws, 0), dev), _bias_autocast(torch.cat(self.bs, 0), dev), self.rows
 
 
 class FluxWeights:
@@ -57,53 +74,46 @@ class FluxWeights:
         w.dim = D = w.heads * w.head_dim
         w.in_channels, w.joint_dim, w.pooled_dim = cfg.in_channels, cfg.joint_attention_dim, cfg.pooled_projection_dim
         w.guidance = bool(cfg.guidance_embeds)
-        w.x_w, w.x_b = _w(m.x_embedder.weight, dev), _b(m.x_embedder.bias, dev)
-        w.ctx_w, w.ctx_b = _w(m.context_embedder.weight, dev), _b(m.context_embedder.bias, dev)
+        w.x_w, w.x_b = _bf16(m.x_embedder.weight, dev), _bias_autocast(m.x_embedder.bias, dev)
+        w.ctx_w, w.ctx_b = _bf16(m.context_embedder.weight, dev), _bias_autocast(m.context_embedder.bias, dev)
         tte = m.time_text_embed
-
-        def mlp(e):
-            return (_w(e.linear_1.weight, dev), _b(e.linear_1.bias, dev), _w(e.linear_2.weight, dev), _b(e.linear_2.bias, dev))
-
-        w.t_mlp, w.p_mlp = mlp(tte.timestep_embedder), mlp(tte.text_embedder)
-        w.g_mlp = mlp(tte.guidance_embedder) if w.guidance else None
-        ada_w, ada_b, off = [], [], 0
-
-        def ada(lin):
-            nonlocal off
-            ada_w.append(lin.weight.detach())
-            ada_b.append(lin.bias.detach())
-            start, off = off, off + lin.weight.shape[0]
-            return start
-
+        w.t_mlp = _mlp2(tte.timestep_embedder.linear_1, tte.timestep_embedder.linear_2, dev)
+        w.p_mlp = _mlp2(tte.text_embedder.linear_1, tte.text_embedder.linear_2, dev)
+        w.g_mlp = _mlp2(tte.guidance_embedder.linear_1, tte.guidance_embedder.linear_2, dev) if w.guidance else None
+        ada = _AdaStack()
         for blk in m.transformer_blocks:
             a = blk.attn
             w.double.append({
-                "ada": ada(blk.norm1.linear), "ada_c": ada(blk.norm1_context.linear),
-                "qk_w": _w(torch.cat([a.to_q.weight, a.to_k.weight], 0), dev), "qk_b": _b(torch.cat([a.to_q.bias, a.to_k.bias], 0), dev),
-                "v_w": _w(a.to_v.weight, dev), "v_b": _b(a.to_v.bias, dev), "o_w": _w(a.to_out[0].weight, dev), "o_b": _b(a.to_out[0].bias, dev),
-                "nq": _b(a.norm_q.weight, dev), "nk": _b(a.norm_k.weight, dev),
-                "cqk_w": _w(torch.cat([a.add_q_proj.weight, a.add_k_proj.weight], 0), dev),
-                "cqk_b": _b(torch.cat([a.add_q_proj.bias, a.add_k_proj.bias], 0), dev),
-                "cv_w": _w(a.add_v_proj.weight, dev), "cv_b": _b(a.add_v_proj.bias, dev),
-                "co_w": _w(a.to_add_out.weight, dev), "co_b": _b(a.to_add_out.bias, dev),
-                "cnq": _b(a.norm_added_q.weight, dev), "cnk": _b(a.norm_added_k.weight, dev),
-                "ff1_w": _w(blk.ff.net[0].proj.weight, dev), "ff1_b": _b(blk.ff.net[0].proj.bias, dev),
-                "ff2_w": _w(blk.ff.net[2].weight, dev), "ff2_b": _b(blk.ff.net[2].bias, dev),
-                "cff1_w": _w(blk.ff_context.net[0].proj.weight, dev), "cff1_b": _b(blk.ff_context.net[0].proj.bias, dev),
-                "cff2_w": _w(blk.ff_context.net[2].weight, dev), "cff2_b": _b(blk.ff_context.net[2].bias, dev),
+                "ada": ada.add(blk.norm1.linear), "ada_c": ada.add(blk.norm1_context.linear),
+                "qk_w": _bf16(torch.cat([a.to_q.weight, a.to_k.weight], 0), dev),
+                "qk_b": _bias_autocast(torch.cat([a.to_q.bias, a.to_k.bias], 0), dev),
+                "v_w": _bf16(a.to_v.weight, dev), "v_b": _bias_autocast(a.to_v.bias, dev),
+                "o_w": _bf16(a.to_out[0].weight, dev), "o_b": _bias_autocast(a.to_out[0].bias, dev),
+                "nq": _bias_autocast(a.norm_q.weight, dev), "nk": _bias_autocast(a.norm_k.weight, dev),
+                "cqk_w": _bf16(torch.cat([a.add_q_proj.weight, a.add_k_proj.weight], 0), dev),
+                "cqk_b": _bias_autocast(torch.cat([a.add_q_proj.bias, a.add_k_proj.bias], 0), dev),
+                "cv_w": _bf16(a.add_v_proj.weight, dev), "cv_b": _bias_autocast(a.add_v_proj.bias, dev),
+                "co_w": _bf16(a.to_add_out.weight, dev), "co_b": _bias_autocast(a.to_add_out.bias, dev),
+                "cnq": _bias_autocast(a.norm_added_q.weight, dev), "cnk": _bias_autocast(a.norm_added_k.weight, dev),
+                "ff1_w": _bf16(blk.ff.net[0].proj.weight, dev), "ff1_b": _bias_autocast(blk.ff.net[0].proj.bias, dev),
+                "ff2_w": _bf16(blk.ff.net[2].weight, dev), "ff2_b": _bias_autocast(blk.ff.net[2].bias, dev),
+                "cff1_w": _bf16(blk.ff_context.net[0].proj.weight, dev), "cff1_b": _bias_autocast(blk.ff_context.net[0].proj.bias, dev),
+                "cff2_w": _bf16(blk.ff_context.net[2].weight, dev), "cff2_b": _bias_autocast(blk.ff_context.net[2].bias, dev),
             })
         for blk in m.single_transformer_blocks:
             a = blk.attn
             w.single.append({
-                "ada": ada(blk.norm.linear),
-                "qk_w": _w(torch.cat([a.to_q.weight, a.to_k.weight], 0), dev), "qk_b": _b(torch.cat([a.to_q.bias, a.to_k.bias], 0), dev),
-                "v_w": _w(a.to_v.weight, dev), "v_b": _b(a.to_v.bias, dev), "nq": _b(a.norm_q.weight, dev), "nk": _b(a.norm_k.weight, dev),
-                "mlp_w": _w(blk.proj_mlp.weight, dev), "mlp_b": _b(blk.proj_mlp.bias, dev),
-                "out_w": _w(blk.proj_out.weight, dev), "out_b": _b(blk.proj_out.bias, dev),
+                "ada": ada.add(blk.norm.linear),
+                "qk_w": _bf16(torch.cat([a.to_q.weight, a.to_k.weight], 0), dev),
+                "qk_b": _bias_autocast(torch.cat([a.to_q.bias, a.to_k.bias], 0), dev),
+                "v_w": _bf16(a.to_v.weight, dev), "v_b": _bias_autocast(a.to_v.bias, dev),
+                "nq": _bias_autocast(a.norm_q.weight, dev), "nk": _bias_autocast(a.norm_k.weight, dev),
+                "mlp_w": _bf16(blk.proj_mlp.weight, dev), "mlp_b": _bias_autocast(blk.proj_mlp.bias, dev),
+                "out_w": _bf16(blk.proj_out.weight, dev), "out_b": _bias_autocast(blk.proj_out.bias, dev),
             })
-        w.ada_out = ada(m.norm_out.linear)
-        w.ada_w, w.ada_b, w.ada_rows = _w(torch.cat(ada_w, 0), dev), _b(torch.cat(ada_b, 0), dev), off
-        w.out_w, w.out_b = _w(m.proj_out.weight, dev), _b(m.proj_out.bias, dev)
+        w.ada_out = ada.add(m.norm_out.linear)
+        w.ada_w, w.ada_b, w.ada_rows = ada.pack(dev)
+        w.out_w, w.out_b = _bf16(m.proj_out.weight, dev), _bias_autocast(m.proj_out.bias, dev)
         w.device = dev
         return w
 
@@ -118,10 +128,18 @@ def rope_table(ids, device, axes_dim=(16, 56, 56), theta=10000.0):
 
 
 class MMDiTCore:
-    """Workspace + block stack shared by the FLUX and HunyuanVideo engines. A subclass provides `self.w` (dim, heads, double, single,
-    ada_w / ada_b / ada_rows), the token order (`txt_first`), the RoPE table of the rows that get RoPE, and its own prologue / head."""
+    """Workspace + block stack shared by the FLUX and HunyuanVideo engines, on the family's packed weights (dim, heads, double,
+    single, ada_w / ada_b / ada_rows). A subclass provides the token order (`txt_first`), the RoPE table of the rows that get RoPE,
+    and its own prologue / head."""
 
     txt_first = True
+
+    def __init__(self, weights, shard_world=1, shard_rank=0, shard_group=None):
+        self.w, self.device = weights, weights.device
+        self.world, self.rank, self.group = shard_world, shard_rank, shard_group
+        self._shape = None
+        self._rope_key, self._rope = None, None
+        self.res_valid = False
 
     def _alloc_core(self, n_img, n_txt):
         """Buffers for one (image tokens, text tokens) shape. Token-sharded (`self.world > 1`, SURVEY §8e): the IMAGE rows are split over
@@ -134,7 +152,7 @@ class MMDiTCore:
         bf = dict(dtype=torch.bfloat16, device=dev)
         self.n_img_total, self.n_txt = n_img, n_txt
         self.shard = None
-        if getattr(self, "world", 1) > 1:
+        if self.world > 1:
             from .shard import TokenShard
             self.shard = TokenShard(self.rank, self.world, n_img, self.group)
             if self.shard.pad:
@@ -324,13 +342,6 @@ class MMDiTCore:
 class FluxEngine(MMDiTCore):
     txt_first = True
 
-    def __init__(self, weights: FluxWeights, shard_world=1, shard_rank=0, shard_group=None):
-        self.w, self.device = weights, weights.device
-        self.world, self.rank, self.group = shard_world, shard_rank, shard_group
-        self._shape = None
-        self._rope_key, self._rope = None, None
-        self.res_valid = False
-
     def _workspace(self, n_img, n_txt):
         if self._shape == (n_img, n_txt):
             return
@@ -412,65 +423,59 @@ class HunyuanWeights:
         if list(m.patch_size) != [1, 2, 2] or m.text_projection != "single_refiner":
             raise NotImplementedError("HunyuanVideo engine: patch (1, 2, 2) and the single_refiner text projection")
         w.in_channels, w.out_channels, w.guidance = m.in_channels, m.out_channels, bool(m.guidance_embed)
-        w.patch_w, w.patch_b = _w(m.img_in.proj.weight.flatten(1), dev), _b(m.img_in.proj.bias, dev)
-
-        def mlp2(a, b_):
-            return (_w(a.weight, dev), _b(a.bias, dev), _w(b_.weight, dev), _b(b_.bias, dev))
-
-        w.t_mlp = mlp2(m.time_in.mlp[0], m.time_in.mlp[2])
-        w.p_mlp = mlp2(m.vector_in.in_layer, m.vector_in.out_layer)
-        w.g_mlp = mlp2(m.guidance_in.mlp[0], m.guidance_in.mlp[2]) if w.guidance else None
+        w.patch_w, w.patch_b = _bf16(m.img_in.proj.weight.flatten(1), dev), _bias_autocast(m.img_in.proj.bias, dev)
+        w.t_mlp = _mlp2(m.time_in.mlp[0], m.time_in.mlp[2], dev)
+        w.p_mlp = _mlp2(m.vector_in.in_layer, m.vector_in.out_layer, dev)
+        w.g_mlp = _mlp2(m.guidance_in.mlp[0], m.guidance_in.mlp[2], dev) if w.guidance else None
         w.pooled_dim = m.vector_in.in_layer.in_features
         r = m.txt_in
         w.text_dim = r.input_embedder.in_features
-        w.r_in_w, w.r_in_b = _w(r.input_embedder.weight, dev), _b(r.input_embedder.bias, dev)
-        w.r_t_mlp = mlp2(r.t_embedder.mlp[0], r.t_embedder.mlp[2])
-        w.r_c_mlp = mlp2(r.c_embedder.linear_1, r.c_embedder.linear_2)
-        r_ada_w, r_ada_b = [], []
+        w.r_in_w, w.r_in_b = _bf16(r.input_embedder.weight, dev), _bias_autocast(r.input_embedder.bias, dev)
+        w.r_t_mlp = _mlp2(r.t_embedder.mlp[0], r.t_embedder.mlp[2], dev)
+        w.r_c_mlp = _mlp2(r.c_embedder.linear_1, r.c_embedder.linear_2, dev)
+        r_ada = _AdaStack()
         for blk in r.individual_token_refiner.blocks:
             W = blk.self_attn_qkv.weight
             Bq = blk.self_attn_qkv.bias
+            r_ada.add(blk.adaLN_modulation[1])
             w.refiner.append({
-                "n1_w": _b(blk.norm1.weight, dev), "n1_b": _b(blk.norm1.bias, dev), "n2_w": _b(blk.norm2.weight, dev), "n2_b": _b(blk.norm2.bias, dev),
-                "qk_w": _w(W[:2 * D], dev), "qk_b": _b(Bq[:2 * D], dev), "v_w": _w(W[2 * D:], dev), "v_b": _b(Bq[2 * D:], dev),
-                "nq": _b(blk.self_attn_q_norm.weight, dev), "nk": _b(blk.self_attn_k_norm.weight, dev),
-                "o_w": _w(blk.self_attn_proj.weight, dev), "o_b": _b(blk.self_attn_proj.bias, dev),
-                "f1_w": _w(blk.mlp.fc1.weight, dev), "f1_b": _b(blk.mlp.fc1.bias, dev), "f2_w": _w(blk.mlp.fc2.weight, dev), "f2_b": _b(blk.mlp.fc2.bias, dev),
+                "n1_w": _bias_autocast(blk.norm1.weight, dev), "n1_b": _bias_autocast(blk.norm1.bias, dev),
+                "n2_w": _bias_autocast(blk.norm2.weight, dev), "n2_b": _bias_autocast(blk.norm2.bias, dev),
+                "qk_w": _bf16(W[:2 * D], dev), "qk_b": _bias_autocast(Bq[:2 * D], dev),
+                "v_w": _bf16(W[2 * D:], dev), "v_b": _bias_autocast(Bq[2 * D:], dev),
+                "nq": _bias_autocast(blk.self_attn_q_norm.weight, dev), "nk": _bias_autocast(blk.self_attn_k_norm.weight, dev),
+                "o_w": _bf16(blk.self_attn_proj.weight, dev), "o_b": _bias_autocast(blk.self_attn_proj.bias, dev),
+                "f1_w": _bf16(blk.mlp.fc1.weight, dev), "f1_b": _bias_autocast(blk.mlp.fc1.bias, dev),
+                "f2_w": _bf16(blk.mlp.fc2.weight, dev), "f2_b": _bias_autocast(blk.mlp.fc2.bias, dev),
             })
-            r_ada_w.append(blk.adaLN_modulation[1].weight.detach())
-            r_ada_b.append(blk.adaLN_modulation[1].bias.detach())
-        w.r_ada_w, w.r_ada_b = _w(torch.cat(r_ada_w, 0), dev), _b(torch.cat(r_ada_b, 0), dev)
-        ada_w, ada_b, off = [], [], 0
-
-        def ada(lin):
-            nonlocal off
-            ada_w.append(lin.weight.detach())
-            ada_b.append(lin.bias.detach())
-            start, off = off, off + lin.weight.shape[0]
-            return start
-
+        w.r_ada_w, w.r_ada_b, _ = r_ada.pack(dev)
+        ada = _AdaStack()
         for blk in m.double_blocks:
-            d = {"ada": ada(blk.img_mod.linear), "ada_c": ada(blk.txt_mod.linear)}
+            d = {"ada": ada.add(blk.img_mod.linear), "ada_c": ada.add(blk.txt_mod.linear)}
             for pre, key in (("img", ""), ("txt", "c")):
                 W, Bq = getattr(blk, f"{pre}_attn_qkv").weight, getattr(blk, f"{pre}_attn_qkv").bias
                 proj, mlp = getattr(blk, f"{pre}_attn_proj"), getattr(blk, f"{pre}_mlp")
-                d.update({f"{key}qk_w": _w(W[:2 * D], dev), f"{key}qk_b": _b(Bq[:2 * D], dev), f"{key}v_w": _w(W[2 * D:], dev), f"{key}v_b": _b(Bq[2 * D:], dev),
-                          f"{key}nq": _b(getattr(blk, f"{pre}_attn_q_norm").weight, dev), f"{key}nk": _b(getattr(blk, f"{pre}_attn_k_norm").weight, dev),
-                          f"{key}o_w": _w(proj.weight, dev), f"{key}o_b": _b(proj.bias, dev),
-                          f"{key}ff1_w": _w(mlp.fc1.weight, dev), f"{key}ff1_b": _b(mlp.fc1.bias, dev),
-                          f"{key}ff2_w": _w(mlp.fc2.weight, dev), f"{key}ff2_b": _b(mlp.fc2.bias, dev)})
+                d.update({f"{key}qk_w": _bf16(W[:2 * D], dev), f"{key}qk_b": _bias_autocast(Bq[:2 * D], dev),
+                          f"{key}v_w": _bf16(W[2 * D:], dev), f"{key}v_b": _bias_autocast(Bq[2 * D:], dev),
+                          f"{key}nq": _bias_autocast(getattr(blk, f"{pre}_attn_q_norm").weight, dev),
+                          f"{key}nk": _bias_autocast(getattr(blk, f"{pre}_attn_k_norm").weight, dev),
+                          f"{key}o_w": _bf16(proj.weight, dev), f"{key}o_b": _bias_autocast(proj.bias, dev),
+                          f"{key}ff1_w": _bf16(mlp.fc1.weight, dev), f"{key}ff1_b": _bias_autocast(mlp.fc1.bias, dev),
+                          f"{key}ff2_w": _bf16(mlp.fc2.weight, dev), f"{key}ff2_b": _bias_autocast(mlp.fc2.bias, dev)})
             w.double.append(d)
         for blk in m.single_blocks:
             W, Bq = blk.linear1.weight, blk.linear1.bias
             w.single.append({
-                "ada": ada(blk.modulation.linear),
-                "qk_w": _w(W[:2 * D], dev), "qk_b": _b(Bq[:2 * D], dev), "v_w": _w(W[2 * D:3 * D], dev), "v_b": _b(Bq[2 * D:3 * D], dev),
-                "mlp_w": _w(W[3 * D:], dev), "mlp_b": _b(Bq[3 * D:], dev), "nq": _b(blk.q_norm.weight, dev), "nk": _b(blk.k_norm.weight, dev),
-                "out_w": _w(blk.linear2.weight, dev), "out_b": _b(blk.linear2.bias, dev),
+                "ada": ada.add(blk.modulation.linear),
+                "qk_w": _bf16(W[:2 * D], dev), "qk_b": _bias_autocast(Bq[:2 * D], dev),
+                "v_w": _bf16(W[2 * D:3 * D], dev), "v_b": _bias_autocast(Bq[2 * D:3 * D], dev),
+                "mlp_w": _bf16(W[3 * D:], dev), "mlp_b": _bias_autocast(Bq[3 * D:], dev),
+                "nq": _bias_autocast(blk.q_norm.weight, dev), "nk": _bias_autocast(blk.k_norm.weight, dev),
+                "out_w": _bf16(blk.linear2.weight, dev), "out_b": _bias_autocast(blk.linear2.bias, dev),
             })
-        w.ada_out = ada(m.final_layer.adaLN_modulation[1])
-        w.ada_w, w.ada_b, w.ada_rows = _w(torch.cat(ada_w, 0), dev), _b(torch.cat(ada_b, 0), dev), off
-        w.out_w, w.out_b = _w(m.final_layer.linear.weight, dev), _b(m.final_layer.linear.bias, dev)
+        w.ada_out = ada.add(m.final_layer.adaLN_modulation[1])
+        w.ada_w, w.ada_b, w.ada_rows = ada.pack(dev)
+        w.out_w, w.out_b = _bf16(m.final_layer.linear.weight, dev), _bias_autocast(m.final_layer.linear.bias, dev)
         w.device = dev
         return w
 
@@ -482,13 +487,9 @@ class HunyuanEngine(MMDiTCore):
 
     txt_first = False
 
-    def __init__(self, weights: HunyuanWeights, shard_world=1, shard_rank=0, shard_group=None):
-        self.w, self.device = weights, weights.device
-        self.world, self.rank, self.group = shard_world, shard_rank, shard_group
-        self._shape = None
-        self._rope_key, self._rope = None, None
+    def __init__(self, weights: HunyuanWeights, **shard_kw):
+        super().__init__(weights, **shard_kw)
         self._mask_key, self._valid = None, None
-        self.res_valid = False
 
     def _workspace(self, grid, n_txt):
         n_img = grid[0] * grid[1] * grid[2]

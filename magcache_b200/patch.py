@@ -19,26 +19,72 @@ import numpy as np
 import torch
 
 from . import ops
-from .config import interp_cfg, table_for_ckpt_dir, tables
+from .config import FAMILIES, interp_cfg, nearest_interp, save_json, table_for_ckpt_dir, table_from_calibration, tables
 from .controller import AttrController
+from .mmdit import FluxEngine, FluxWeights, HunyuanEngine, HunyuanWeights
 from .wan import WanEngine, WanWeights
 
-_WAN_CTRL = dict(branches=2, cmp=0, retention_mode=0, veto_index=-1, veto_base=0)  # `<`, int(n*R): magcache_generate.py:279-286
+
+def _cached_engine(self, attr, engine_cls, make_weights):
+    """The engine cached on the model under `attr`, built on first use from `make_weights()` (token-sharded when
+    `enable_token_shard` was called)."""
+    eng = self.__dict__.get(attr)
+    if eng is None:
+        eng = engine_cls(make_weights(), **self.__dict__.get("_mc_shard_kw", {}))
+        object.__setattr__(self, attr, eng)
+    return eng
+
+
+def _wan_weights(self):
+    if not hasattr(self, "patch_embedding"):
+        raise TypeError("magcache_b200.magcache_forward expects a Wan2.1 WanModel (or an object carrying `_mc_engine`)")
+    dev = self.patch_embedding.weight.device
+    if dev.type != "cuda":
+        raise RuntimeError("magcache_b200: the model must be on a CUDA device (no CPU path)")
+    return WanWeights.from_module(self, dev)
 
 
 def _engine(self):
-    eng = self.__dict__.get("_mc_engine")
-    if eng is None:
-        if hasattr(self, "patch_embedding"):
-            dev = self.patch_embedding.weight.device
-            if dev.type != "cuda":
-                raise RuntimeError("magcache_b200: the model must be on a CUDA device (no CPU path)")
-            weights = WanWeights.from_module(self, dev)
-        else:
-            raise TypeError("magcache_b200.magcache_forward expects a Wan2.1 WanModel (or an object carrying `_mc_engine`)")
-        eng = WanEngine(weights, **self.__dict__.get("_mc_shard_kw", {}))
-        object.__setattr__(self, "_mc_engine", eng)
-    return eng
+    return _cached_engine(self, "_mc_engine", WanEngine, lambda: _wan_weights(self))
+
+
+def _family_controller(self, family):
+    """The skip controller of `family` (a key of `config.FAMILIES`) for this model, created on first use."""
+    ctrls = self.__dict__.setdefault("_mc_ctrls", {})
+    if family not in ctrls:
+        ctrls[family] = AttrController(FAMILIES[family])
+    return ctrls[family]
+
+
+def _adopt_residual(cur, buf, valid):
+    """The reference keeps the cached residual in a model attribute (`cur`); the engine keeps it in a fixed buffer `buf` that the
+    attribute aliases. If a caller replaced the attribute, copy it in; if they cleared it, the buffer is empty. Returns the buffer's
+    new validity (`valid`: its current one)."""
+    if cur is None:
+        return False
+    if torch.is_tensor(cur) and cur.data_ptr() != buf.data_ptr():
+        buf.copy_(cur.reshape(buf.shape))
+        return True
+    return valid
+
+
+def _record_stats(self, stats):
+    """Append the calibration statistics of one call, rounded to 5 places, and print the reference's per-call line
+    (MagCache4Wan2.1/magcache_generate.py:170-173 ; magcache_flux.py:202-205 ; magcache_sample_video.py:258-261)."""
+    norm_ratio, norm_std, cos_dis = stats
+    self.norm_ratio.append(round(norm_ratio, 5))
+    self.norm_std.append(round(norm_std, 5))
+    self.cos_dis.append(round(cos_dis, 5))
+    print(f"time: {self.cnt}, norm_ratio: {norm_ratio}, norm_std: {norm_std}, cos_dis: {cos_dis}")
+
+
+def _print_stats(self):
+    print("norm ratio")
+    print(self.norm_ratio)
+    print("norm std")
+    print(self.norm_std)
+    print("cos_dis")
+    print(self.cos_dis)
 
 
 def invalidate_engine(model):
@@ -46,7 +92,7 @@ def invalidate_engine(model):
     graphs). The engine snapshots the module's parameters at the first forward: call this after anything that changes them — a LoRA
     merge, `load_state_dict`, `.to(...)` — and the next forward repacks. The module's own parameters stay resident next to the
     packed copy (about +2.8 GB for the 1.3B model, +28 GB for 14B); free or offload them yourself if that matters."""
-    for name in ("_mc_engine", "_mc_flux_engine", "_mc_hunyuan_engine", "_mc_ctrl"):
+    for name in ("_mc_engine", "_mc_flux_engine", "_mc_hunyuan_engine", "_mc_ctrls"):
         model.__dict__.pop(name, None)
     return model
 
@@ -62,15 +108,7 @@ def enable_token_shard(model, rank, world, group=None):
     return model
 
 
-def _controller(self):
-    c = self.__dict__.get("_mc_ctrl")
-    if c is None:
-        c = AttrController(_WAN_CTRL)
-        object.__setattr__(self, "_mc_ctrl", c)
-    return c
-
-
-def _stage(self, x, t, context, seq_len, clip_fea, y, pad_ok=True, vace_context=None, vace_scale=1.0, require_clip=True):
+def _stage(self, x, t, context, seq_len, clip_fea, y, calibration=False, vace_context=None, vace_scale=1.0, require_clip=True):
     if getattr(self, "model_type", "t2v") == "i2v" and require_clip:
         assert clip_fea is not None and y is not None  # magcache_generate.py:226-227
     if len(x) != 1 or len(context) != 1 or (y is not None and len(y) != 1):
@@ -84,39 +122,26 @@ def _stage(self, x, t, context, seq_len, clip_fea, y, pad_ok=True, vace_context=
     # seq_len > n_tok (upstream rounds seq_len up to a multiple of the sequence-parallel size): the reference appends zero rows
     # (:243-246) that never reach a real token — keys are masked by k_lens = seq_lens, every other op is per token, unpatchify
     # reads the first n_tok rows — so the forwards simply do not compute them; the only visible difference: residual_cache[i] has
-    # n_tok rows instead of seq_len. The calibration statistics DO average over the padded rows upstream: there (pad_ok=False) ONE
-    # representative pad row is computed — the padded rows are all identical — and weighted by their count.
-    pad_row = 1 if (n_tok != seq_len and pad_ok is False) else 0
+    # n_tok rows instead of seq_len. The calibration statistics DO average over the padded rows upstream: there ONE representative
+    # pad row is computed — the padded rows are all identical — and weighted by their count.
     if vace_context is not None and len(vace_context) != 1:
         raise NotImplementedError("magcache_b200: one sample per call")
     eng.stage_inputs(lat, t, context[0], clip_fea=clip_fea, y=None if y is None else y[0],
-                     vace_context=None if vace_context is None else vace_context[0], vace_scale=vace_scale, pad_row=pad_row)
-    eng.pad_weight = (seq_len - n_tok) if pad_row else 0
+                     vace_context=None if vace_context is None else vace_context[0], vace_scale=vace_scale,
+                     n_pad=seq_len - n_tok if calibration else 0)
     return eng
 
 
-def _sync_slot_in(self, eng, slot):
-    """The reference keeps the cached residual in `self.residual_cache[slot]`; the engine keeps it in a fixed buffer that the
-    attribute aliases. If a caller replaced the attribute (or cleared it), follow the attribute."""
-    cur = self.residual_cache[slot]
-    if cur is None:
-        eng.res_valid[slot] = False
-    elif torch.is_tensor(cur) and cur.data_ptr() != eng.res[slot].data_ptr():
-        eng.res[slot].copy_(cur.reshape(eng.res[slot].shape))
-        eng.res_valid[slot] = True
-
-
-def magcache_forward(self, x, t, context, seq_len, clip_fea=None, y=None):
-    r"""MagCache4Wan2.1/magcache_generate.py:198-312 on the B200 kernels.
-
-    Args / returns as the reference: x List[Tensor[C_in, F, H, W]], t Tensor[B], context List[Tensor[L, C]], seq_len int
-    -> List[Tensor[C_out, F, H, W]] (float32).
-    """
-    eng = _stage(self, x, t, context, seq_len, clip_fea, y)
-    ctrl = _controller(self)
-    slot = self.cnt % 2
-    skip_forward = ctrl.decide(self)  # :279-292 (float64 state under the reference's attribute names)
-    _sync_slot_in(self, eng, slot)
+def _wan_cached_step(self, eng, family, print_skip=False):
+    """One cached Wan forward on staged inputs (MagCache4Wan2.1/magcache_generate.py:277-311; VACE :517-559; Wan2.2
+    MagCache4Wan2.2/magcache_generate.py:290-334): decide, follow the residual attribute, hit or miss, store the residual, advance."""
+    ctrl = _family_controller(self, family)
+    slot = int(self.cnt) % 2
+    skip_forward = ctrl.decide(self)  # float64 state under the reference's attribute names
+    # Wan2.2: the other expert's residual arrives through the class-level list the two experts share
+    eng.res_valid[slot] = _adopt_residual(self.residual_cache[slot], eng.res[slot], eng.res_valid[slot])
+    if print_skip and skip_forward:
+        print("skip: ", self.cnt)  # VACE, :527
     # hit : `x = x + residual_x` (:295) feeds only the head, so the sum is formed inside the head kernel (same fp32 arithmetic)
     # miss: block stack (:297-298), `residual_x = x - ori_x` (:299) written into the slot's buffer
     out = eng.forward("hit" if skip_forward else "miss", slot)
@@ -125,27 +150,27 @@ def magcache_forward(self, x, t, context, seq_len, clip_fea=None, y=None):
     return [out]
 
 
+def magcache_forward(self, x, t, context, seq_len, clip_fea=None, y=None):
+    r"""MagCache4Wan2.1/magcache_generate.py:198-312 on the B200 kernels.
+
+    Args / returns as the reference: x List[Tensor[C_in, F, H, W]], t Tensor[B], context List[Tensor[L, C]], seq_len int
+    -> List[Tensor[C_out, F, H, W]] (float32).
+    """
+    return _wan_cached_step(self, _stage(self, x, t, context, seq_len, clip_fea, y), "wan2.1")
+
+
 def magcache_vace_forward(self, x, t, vace_context, context, seq_len, vace_context_scale=1.0, clip_fea=None, y=None):
     r"""MagCache4Wan2.1/magcache_generate.py:439-560 (installed at :1126-1150 with the VACE tables): the T2V forward plus the
     control branch. `vace_context`: List[Tensor[96, F, H, W]]. On a miss the control blocks run first (`forward_vace`, :541) and
     every second main block adds its hint; on a hit nothing of the control branch is computed, as in the reference. `clip_fea` and
     `y` are accepted and ignored (the reference has those lines commented out, :471-476, :505-507)."""
     eng = _stage(self, x, t, context, seq_len, None, None, vace_context=vace_context, vace_scale=vace_context_scale)
-    ctrl = _controller(self)
-    slot = self.cnt % 2
-    skip_forward = ctrl.decide(self)  # :517-531
-    _sync_slot_in(self, eng, slot)
-    if skip_forward:
-        print("skip: ", self.cnt)  # :527
-    out = eng.forward("hit" if skip_forward else "miss", slot)
-    self.residual_cache[slot] = eng.res[slot].view(1, *eng.res[slot].shape)  # :549
-    ctrl.advance(self)  # :554-559
-    return [out]
+    return _wan_cached_step(self, eng, "wan2.1", print_skip=True)  # :517-559
 
 
 def magcache_vace_calibration(self, x, t, vace_context, context, seq_len, vace_context_scale=1.0, clip_fea=None, y=None):
     r"""MagCache4Wan2.1/magcache_generate.py:314-436: `magcache_calibration` with the control branch."""
-    return _calibrate(self, _stage(self, x, t, context, seq_len, None, None, pad_ok=False, vace_context=vace_context,
+    return _calibrate(self, _stage(self, x, t, context, seq_len, None, None, calibration=True, vace_context=vace_context,
                                    vace_scale=vace_context_scale))
 
 
@@ -164,26 +189,13 @@ def magcache_wan22_forward(self, x, t, context, seq_len, clip_fea=None, y=None):
             raise NotImplementedError("magcache_b200: one sample per call")
         assert t.size(1) == seq_len  # what `.unflatten(0, (bt, seq_len))` (:270) requires
     eng = _stage(self, x, t, context, seq_len, None, y, require_clip=False)
-    ctrls = self.__dict__.setdefault("_mc_ctrls", {})
-    fam = "wan2.2-i2v" if getattr(self, "mode", "t2v") == "i2v" else "wan2.2-t2v"
-    if fam not in ctrls:
-        from .config import FAMILIES
-        ctrls[fam] = AttrController(FAMILIES[fam])
-    ctrl = ctrls[fam]
-    slot = int(self.cnt) % 2
-    skip_forward = ctrl.decide(self)  # :290-317
-    _sync_slot_in(self, eng, slot)    # the other expert's residual arrives through the shared class-level list
-    out = eng.forward("hit" if skip_forward else "miss", slot)
-    self.residual_cache[slot] = eng.res[slot].view(1, *eng.res[slot].shape)  # :324
-    ctrl.advance(self)  # :328-334
-    return [out]
+    return _wan_cached_step(self, eng, "wan2.2-i2v" if getattr(self, "mode", "t2v") == "i2v" else "wan2.2-t2v")  # :290-334
 
 
 def init_magcache_wan22(model, mag_ratios, sample_steps, thresh=0.06, K=2, retention_ratio=0.2, split_steps=None, mode="t2v"):
     """`init_magcache(model, mag_ratios, args, split_steps, mode)` of MagCache4Wan2.2/magcache_generate.py:340-362: patches the CLASS the
     two experts share. `mag_ratios`: the list without its `[1.0]*2` prefix like the script passes it, or a key of `tables()` (which
     already carries the prefix)."""
-    import numpy as np
     cls = model.__class__
     cls.forward = magcache_wan22_forward
     cls.cnt = torch.tensor(0)
@@ -202,56 +214,26 @@ def init_magcache_wan22(model, mag_ratios, sample_steps, thresh=0.06, K=2, reten
 def magcache_calibration(self, x, t, context, seq_len, clip_fea=None, y=None):
     r"""MagCache4Wan2.1/magcache_generate.py:80-194: always runs the block stack and records, per forward, the token-mean
     magnitude ratio, its std and the cosine distance to the previous residual of the same CFG branch (one fused pass)."""
-    return _calibrate(self, _stage(self, x, t, context, seq_len, clip_fea, y, pad_ok=False))
+    return _calibrate(self, _stage(self, x, t, context, seq_len, clip_fea, y, calibration=True))
 
 
 def _calibrate(self, eng):
-    x0, e, e0, ctx = eng.prologue()
-    xs = eng.run_blocks(x0, e0, ctx, eng.grid)
     slot = self.cnt % 2
-    if self.cnt >= 2:
-        prev = self.residual_cache[slot].view(x0.shape)
-        reduce = None
-        if eng.shard is not None:  # the statistics are sums over tokens: add the partial sums of every token shard
-            from .shard import allreduce_stats
-            reduce = lambda st: allreduce_stats(st, eng.shard.group)  # noqa: E731
-        if eng.pad_row:
-            # seq_len > token count: rows [n_tok, seq_len) of the reference's tensors are identical copies of the one pad row computed
-            # here; its three per-row terms enter the means (seq_len - n_tok) times (:167-169 average over dim 1 of [1, seq_len, D])
-            n_tok, wgt = eng.n_keys, float(eng.pad_weight)
-            keep = {}
-            ops.residual_sub_stats(xs[n_tok:], x0[n_tok:], prev[n_tok:].contiguous(), reduce=lambda st: keep.setdefault("pad", st.clone()))
-            residual_tok, (norm_ratio, norm_std, cos_dis) = ops.residual_sub_stats(
-                xs[:n_tok], x0[:n_tok], prev[:n_tok].contiguous(), reduce=lambda st: st + keep["pad"] * st.new_tensor([wgt, wgt, wgt, wgt]))
-            residual_x = torch.cat([residual_tok, xs[n_tok:] - x0[n_tok:].float()])
-        else:
-            residual_x, (norm_ratio, norm_std, cos_dis) = ops.residual_sub_stats(xs, x0, prev, reduce=reduce)
-        self.norm_ratio.append(round(norm_ratio, 5))
-        self.norm_std.append(round(norm_std, 5))
-        self.cos_dis.append(round(cos_dis, 5))
-        print(f"time: {self.cnt}, norm_ratio: {norm_ratio}, norm_std: {norm_std}, cos_dis: {cos_dis}")
-    else:
-        residual_x = ops.residual_sub(xs, x0)
-    self.residual_cache[slot] = residual_x.view(1, *x0.shape)
-    eng._slot = slot
-    out = eng.head(xs, e, eng.grid)
+    out, residual, stats = eng.calibrate(slot, self.residual_cache[slot] if self.cnt >= 2 else None)  # :163-175
+    if stats is not None:
+        _record_stats(self, stats)
+    self.residual_cache[slot] = residual.view(1, *residual.shape)
     self.cnt += 1
-    if self.cnt >= self.num_steps:
+    if self.cnt >= self.num_steps:  # :180-193: the lists are printed and saved at the wrap
         self.cnt = 0
         self.accumulated_ratio = [1.0, 1.0]
         self.accumulated_err = [0.0, 0.0]
         self.accumulated_steps = [0, 0]
-        print("norm ratio")
-        print(self.norm_ratio)
-        print("norm std")
-        print(self.norm_std)
-        print("cos_dis")
-        print(self.cos_dis)
+        _print_stats(self)
         # :191-193 `save_json("wan2_1_mag_ratio", self.norm_ratio)` ...: same file names, in `calibration_dir` (default: the
         # working directory, like the reference). `config.table_from_calibration` turns the first file into a `mag_ratios` table.
         out_dir = getattr(self, "calibration_dir", ".")
         if out_dir is not None:
-            from .config import save_json
             save_json(os.path.join(out_dir, "wan2_1_mag_ratio"), self.norm_ratio)
             save_json(os.path.join(out_dir, "wan2_1_mag_std"), self.norm_std)
             save_json(os.path.join(out_dir, "wan2_1_cos_dis"), self.cos_dis)
@@ -274,7 +256,6 @@ def init_magcache(model, sample_steps, thresh=0.12, K=2, retention_ratio=0.2, ma
     cls.retention_ratio = retention_ratio
     cls.residual_cache = [None, None]
     if isinstance(mag_ratios, (str, os.PathLike)):  # a calibration dump (`wan2_1_mag_ratio.json`) instead of a pasted literal
-        from .config import table_from_calibration
         mag_ratios = table_from_calibration(mag_ratios)
     if mag_ratios is None:
         mag_ratios = tables()[table] if table is not None else table_for_ckpt_dir(ckpt_dir)
@@ -318,11 +299,7 @@ def magcache_branch(self, hidden, run_blocks, family, cache_attr):
     the cached residual (K1 kernel) or calls `run_blocks(hidden)` (the model's own transformer stack) and stores `out - hidden`
     (K2 kernel) under `cache_attr` — a tensor for scalar-state families, a 2-list indexed by `cnt % 2` for per-branch ones.
     Advances the counter. Wan2.2's expert boundary is read from `self.split_step` like upstream (:344)."""
-    from .config import FAMILIES
-    ctrls = self.__dict__.setdefault("_mc_ctrls", {})
-    if family not in ctrls:
-        ctrls[family] = AttrController(FAMILIES[family])
-    ctrl = ctrls[family]
+    ctrl = _family_controller(self, family)
     per_branch = FAMILIES[family]["branches"] == 2
     slot = int(self.cnt) % 2 if per_branch else None
     if ctrl.decide(self):
@@ -342,7 +319,7 @@ def magcache_branch(self, hidden, run_blocks, family, cache_attr):
 
 
 # ------------------------------------------------------------------------------------------------------------------
-# FLUX: the whole patched forward on the MMDiT engine (magcache_b200/flux.py; opt-in until validated on a GPU, see its header)
+# FLUX and HunyuanVideo: the whole patched forward on the MMDiT engines (magcache_b200/mmdit.py)
 # ------------------------------------------------------------------------------------------------------------------
 class _Sample:
     """Stand-in for diffusers' Transformer2DModelOutput (`.sample`), which is not importable here."""
@@ -351,50 +328,55 @@ class _Sample:
         self.sample = sample
 
 
+def _mmdit_cached_step(self, eng, family, res_attr):
+    """One cached MMDiT forward on staged inputs (magcache_flux.py:326-436 ; magcache_sample_video.py:88-154): decide, follow the
+    residual attribute `res_attr`, hit or miss, store the residual, advance. Returns the engine's output."""
+    ctrl = _family_controller(self, family)
+    skip_forward = ctrl.decide(self)
+    eng.res_valid = _adopt_residual(getattr(self, res_attr), eng.res, eng.res_valid)
+    out = eng.forward("hit" if skip_forward else "miss")
+    setattr(self, res_attr, eng.res.view(1, *eng.res.shape))  # :427 ; :141
+    ctrl.advance(self)
+    return out
+
+
+def _mmdit_calibration_step(self, eng, res_attr):
+    """One MMDiT calibration call on staged inputs: block stack, statistics from the second call of a generation on, residual
+    stored under `res_attr`. Returns the engine's output."""
+    if self.cnt == 0:
+        eng.res_valid = False  # `if self.cnt>=1` (magcache_flux.py:198 ; magcache_sample_video.py:254): nothing to compare with
+    out, stats = eng.calibrate()
+    if stats is not None:
+        _record_stats(self, stats)
+    setattr(self, res_attr, eng.res.view(1, *eng.res.shape))
+    return out
+
+
+def _flux_stage(self, hidden_states, encoder_hidden_states, pooled_projections, timestep, img_ids, txt_ids, guidance,
+                joint_attention_kwargs, controlnet_block_samples, controlnet_single_block_samples):
+    if joint_attention_kwargs or controlnet_block_samples is not None or controlnet_single_block_samples is not None:
+        raise NotImplementedError("magcache_b200: joint_attention_kwargs / ControlNet residuals are not built for the FLUX engine")
+    if not hidden_states.is_cuda:
+        raise RuntimeError("magcache_b200: hidden_states must be CUDA tensors (no CPU path)")
+    eng = _cached_engine(self, "_mc_flux_engine", FluxEngine, lambda: FluxWeights.from_module(self, hidden_states.device))
+    eng.stage_inputs(hidden_states, encoder_hidden_states, pooled_projections, timestep, guidance,
+                     img_ids[0] if img_ids.ndim == 3 else img_ids, txt_ids[0] if txt_ids.ndim == 3 else txt_ids)  # :305-316 (3-D ids)
+    return eng
+
+
 def magcache_flux_forward(self, hidden_states, encoder_hidden_states=None, pooled_projections=None, timestep=None, img_ids=None,
                           txt_ids=None, guidance=None, joint_attention_kwargs=None, controlnet_block_samples=None,
                           controlnet_single_block_samples=None, return_dict=True, controlnet_blocks_repeat=False):
     r"""MagCache4FLUX/magcache_flux.py:234-440 on the B200 kernels: same signature, same state attributes (`cnt, num_steps,
     magcache_thresh, K, retention_ratio, accumulated_ratio / _err / _steps, previous_residual, mag_ratios`), `(output,)` or an object
     with `.sample`. LoRA scaling, ip-adapter and ControlNet residuals (:275-288, :321-324, :371-381, :410-420) are not built and raise."""
-    if joint_attention_kwargs or controlnet_block_samples is not None or controlnet_single_block_samples is not None:
-        raise NotImplementedError("magcache_b200: joint_attention_kwargs / ControlNet residuals are not built for the FLUX engine")
-    if not hidden_states.is_cuda:
-        raise RuntimeError("magcache_b200: hidden_states must be CUDA tensors (no CPU path)")
-    eng = _flux_engine(self, hidden_states)
-    if txt_ids.ndim == 3:  # :305-316 (deprecated 3-D ids)
-        txt_ids = txt_ids[0]
-    if img_ids.ndim == 3:
-        img_ids = img_ids[0]
-    eng.stage_inputs(hidden_states, encoder_hidden_states, pooled_projections, timestep, guidance, img_ids, txt_ids)
-    ctrls = self.__dict__.setdefault("_mc_ctrls", {})
-    if "flux" not in ctrls:
-        from .config import FAMILIES
-        ctrls["flux"] = AttrController(FAMILIES["flux"])
-    ctrl = ctrls["flux"]
-    skip_forward = ctrl.decide(self)  # :326-338
-    cur = self.previous_residual
-    if cur is None:
-        eng.res_valid = False
-    elif torch.is_tensor(cur) and cur.data_ptr() != eng.res.data_ptr():
-        eng.res.copy_(cur.reshape(eng.res.shape))
-        eng.res_valid = True
-    out = eng.forward("hit" if skip_forward else "miss")
-    self.previous_residual = eng.res.view(1, *eng.res.shape)  # :427
-    ctrl.advance(self)  # :431-436
+    eng = _flux_stage(self, hidden_states, encoder_hidden_states, pooled_projections, timestep, img_ids, txt_ids, guidance,
+                      joint_attention_kwargs, controlnet_block_samples, controlnet_single_block_samples)
+    out = _mmdit_cached_step(self, eng, "flux", "previous_residual")
     output = out.view(1, *out.shape)
     if not return_dict:
         return (output,)
     return _Sample(output)
-
-
-def _flux_engine(self, hidden_states):
-    eng = self.__dict__.get("_mc_flux_engine")
-    if eng is None:
-        from .mmdit import FluxEngine, FluxWeights
-        eng = FluxEngine(FluxWeights.from_module(self, hidden_states.device), **self.__dict__.get("_mc_shard_kw", {}))
-        object.__setattr__(self, "_mc_flux_engine", eng)
-    return eng
 
 
 def magcache_flux_calibration(self, hidden_states, encoder_hidden_states=None, pooled_projections=None, timestep=None, img_ids=None,
@@ -403,32 +385,13 @@ def magcache_flux_calibration(self, hidden_states, encoder_hidden_states=None, p
     r"""MagCache4FLUX/magcache_flux.py:21-231: every call runs the block stack and, from the second call on, records the token-mean
     magnitude ratio, its std and the cosine distance to the previous residual (`norm_ratio / norm_std / cos_dis`, rounded to 5 places);
     the lists are printed on the last call of a generation and cleared at the wrap (:207-221)."""
-    if joint_attention_kwargs or controlnet_block_samples is not None or controlnet_single_block_samples is not None:
-        raise NotImplementedError("magcache_b200: joint_attention_kwargs / ControlNet residuals are not built for the FLUX engine")
-    if not hidden_states.is_cuda:
-        raise RuntimeError("magcache_b200: hidden_states must be CUDA tensors (no CPU path)")
-    eng = _flux_engine(self, hidden_states)
-    eng.stage_inputs(hidden_states, encoder_hidden_states, pooled_projections, timestep, guidance,
-                     img_ids[0] if img_ids.ndim == 3 else img_ids, txt_ids[0] if txt_ids.ndim == 3 else txt_ids)
-    if self.cnt == 0:
-        eng.res_valid = False  # `if self.cnt>=1` (:199): the first call of a generation has nothing to compare with
-    out, stats = eng.calibrate()
-    if self.cnt >= 1 and stats is not None:
-        norm_ratio, norm_std, cos_dis = stats
-        self.norm_ratio.append(round(norm_ratio, 5))
-        self.norm_std.append(round(norm_std, 5))
-        self.cos_dis.append(round(cos_dis, 5))
-        print(f"time: {self.cnt}, norm_ratio: {norm_ratio}, norm_std: {norm_std}, cos_dis: {cos_dis}")
-    self.previous_residual = eng.res.view(1, *eng.res.shape)
-    if self.cnt >= self.num_steps - 1:
-        print("norm ratio")
-        print(self.norm_ratio)
-        print("norm std")
-        print(self.norm_std)
-        print("cos_dis")
-        print(self.cos_dis)
+    eng = _flux_stage(self, hidden_states, encoder_hidden_states, pooled_projections, timestep, img_ids, txt_ids, guidance,
+                      joint_attention_kwargs, controlnet_block_samples, controlnet_single_block_samples)
+    out = _mmdit_calibration_step(self, eng, "previous_residual")
+    if self.cnt >= self.num_steps - 1:  # :207-213
+        _print_stats(self)
     self.cnt += 1
-    if self.cnt >= self.num_steps:
+    if self.cnt >= self.num_steps:  # :219-222
         self.cnt = 0
         self.norm_ratio, self.norm_std, self.cos_dis = [], [], []
     output = out.view(1, *out.shape)
@@ -448,8 +411,6 @@ def init_magcache_flux_calibration(transformer, num_inference_steps=28):
 def init_magcache_flux(transformer, num_inference_steps=28, thresh=0.24, K=5, retention_ratio=0.1, mag_ratios=None, table="flux_dev"):
     """The installation statements of magcache_flux.py:446-471 (Kontext: magcache_flux_kontext.py:445-470 with table "flux_kontext",
     thresh 0.05, K 4, retention 0.2): patches the CLASS."""
-    from .config import nearest_interp
-    import numpy as np
     cls = transformer.__class__
     cls.forward = magcache_flux_forward
     cls.cnt, cls.num_steps = 0, num_inference_steps
@@ -463,35 +424,22 @@ def init_magcache_flux(transformer, num_inference_steps=28, thresh=0.24, K=5, re
     return transformer
 
 
-def magcache_hunyuan_forward(self, x, t, text_states=None, text_mask=None, text_states_2=None, freqs_cos=None, freqs_sin=None,
-                             guidance=None, return_dict=True):
-    r"""MagCache4HunyuanVideo/magcache_sample_video.py:29-160 on the B200 kernels (MMDiT engine, magcache_b200/mmdit.py; opt-in until
-    validated on a GPU): same signature and state attributes (`cnt, num_steps, magcache_thresh, K, retention_ratio, accumulated_ratio /
-    _err / _steps, residual_cache, mag_ratios`), returns `{"x": img}` or the tensor. x [1, 16, T, H, W]; text_mask marks the valid
-    (right-padded) text tokens."""
+def _hunyuan_stage(self, x, t, text_states, text_mask, text_states_2, freqs_cos, freqs_sin, guidance):
     if not x.is_cuda:
         raise RuntimeError("magcache_b200: x must be a CUDA tensor (no CPU path)")
-    eng = self.__dict__.get("_mc_hunyuan_engine")
-    if eng is None:
-        from .mmdit import HunyuanEngine, HunyuanWeights
-        eng = HunyuanEngine(HunyuanWeights.from_module(self, x.device), **self.__dict__.get("_mc_shard_kw", {}))
-        object.__setattr__(self, "_mc_hunyuan_engine", eng)
+    eng = _cached_engine(self, "_mc_hunyuan_engine", HunyuanEngine, lambda: HunyuanWeights.from_module(self, x.device))
     eng.stage_inputs(x, t, text_states, text_mask, text_states_2, freqs_cos, freqs_sin, guidance)
-    ctrls = self.__dict__.setdefault("_mc_ctrls", {})
-    if "hunyuan" not in ctrls:
-        from .config import FAMILIES
-        ctrls["hunyuan"] = AttrController(FAMILIES["hunyuan"])
-    ctrl = ctrls["hunyuan"]
-    skip_forward = ctrl.decide(self)  # :88-102
-    cur = self.residual_cache
-    if cur is None:
-        eng.res_valid = False
-    elif torch.is_tensor(cur) and cur.data_ptr() != eng.res.data_ptr():
-        eng.res.copy_(cur.reshape(eng.res.shape))
-        eng.res_valid = True
-    img = eng.forward("hit" if skip_forward else "miss")
-    self.residual_cache = eng.res.view(1, *eng.res.shape)  # :141
-    ctrl.advance(self)  # :149-154
+    return eng
+
+
+def magcache_hunyuan_forward(self, x, t, text_states=None, text_mask=None, text_states_2=None, freqs_cos=None, freqs_sin=None,
+                             guidance=None, return_dict=True):
+    r"""MagCache4HunyuanVideo/magcache_sample_video.py:29-160 on the B200 kernels (MMDiT engine, magcache_b200/mmdit.py): same
+    signature and state attributes (`cnt, num_steps, magcache_thresh, K, retention_ratio, accumulated_ratio / _err / _steps,
+    residual_cache, mag_ratios`), returns `{"x": img}` or the tensor. x [1, 16, T, H, W]; text_mask marks the valid (right-padded)
+    text tokens."""
+    eng = _hunyuan_stage(self, x, t, text_states, text_mask, text_states_2, freqs_cos, freqs_sin, guidance)
+    img = _mmdit_cached_step(self, eng, "hunyuan", "residual_cache")
     if return_dict:
         return {"x": img}
     return img
@@ -500,32 +448,11 @@ def magcache_hunyuan_forward(self, x, t, text_states=None, text_mask=None, text_
 def magcache_hunyuan_calibration(self, x, t, text_states=None, text_mask=None, text_states_2=None, freqs_cos=None, freqs_sin=None,
                                  guidance=None, return_dict=True):
     r"""MagCache4HunyuanVideo/magcache_sample_video.py:163-290: the calibration twin (statistics from the second call on, lists printed
-    from call 49 on — hard-coded upstream, :266 — and a counter that is never wrapped, :281)."""
-    if not x.is_cuda:
-        raise RuntimeError("magcache_b200: x must be a CUDA tensor (no CPU path)")
-    eng = self.__dict__.get("_mc_hunyuan_engine")
-    if eng is None:
-        from .mmdit import HunyuanEngine, HunyuanWeights
-        eng = HunyuanEngine(HunyuanWeights.from_module(self, x.device))
-        object.__setattr__(self, "_mc_hunyuan_engine", eng)
-    eng.stage_inputs(x, t, text_states, text_mask, text_states_2, freqs_cos, freqs_sin, guidance)
-    if self.cnt == 0:
-        eng.res_valid = False
-    img, stats = eng.calibrate()
-    if self.cnt >= 1 and stats is not None:
-        norm_ratio, norm_std, cos_dis = stats
-        self.norm_ratio.append(round(norm_ratio, 5))
-        self.norm_std.append(round(norm_std, 5))
-        self.cos_dis.append(round(cos_dis, 5))
-        print(f"time: {self.cnt}, norm_ratio: {norm_ratio}, norm_std: {norm_std}, cos_dis: {cos_dis}")
-    self.residual_cache = eng.res.view(1, *eng.res.shape)
-    if self.cnt >= 49:
-        print("norm ratio")
-        print(self.norm_ratio)
-        print("norm std")
-        print(self.norm_std)
-        print("cos_dis")
-        print(self.cos_dis)
+    from call 49 on — hard-coded upstream, :264 — and a counter that is never wrapped, :277)."""
+    eng = _hunyuan_stage(self, x, t, text_states, text_mask, text_states_2, freqs_cos, freqs_sin, guidance)
+    img = _mmdit_calibration_step(self, eng, "residual_cache")
+    if self.cnt >= 49:  # :264-270
+        _print_stats(self)
     self.cnt += 1
     return {"x": img} if return_dict else img
 
@@ -542,9 +469,6 @@ def init_magcache_hunyuan_calibration(transformer, infer_steps=50):
 
 def init_magcache_hunyuan(transformer, infer_steps=50, thresh=0.24, K=6, retention_ratio=0.2, video_height=720, mag_ratios=None):
     """The installation statements of magcache_sample_video.py:303-328 (table chosen by `args.video_size[0]` in {720, 544}, :315-318)."""
-    import numpy as np
-
-    from .config import nearest_interp
     cls = transformer.__class__
     cls.cnt, cls.num_steps, cls.magcache_thresh, cls.K = 0, infer_steps, thresh, K
     cls.residual_cache = None
@@ -574,7 +498,6 @@ def magcache_eval_forward(self, x, t, context, seq_len, clip_fea=None, y=None):
     import ctypes
 
     from . import _lib
-    from .config import FAMILIES
     from .controller import make_ctrl_config
     eng = _stage(self, x, t, context, seq_len, clip_fea, y)
     cache_time = 10                                  # :771
@@ -615,7 +538,6 @@ def magcache_eval_forward(self, x, t, context, seq_len, clip_fea=None, y=None):
 
 def init_magcache_eval(model, sample_steps, thresh=0.12, K=2, ratio=None):
     """The installation block of wan_magcache.py:1129-1150 as a helper ("slow" = 0.12/K2, "fast" = 0.12/K4, wan_eval.sh:30-31,66-67)."""
-    import numpy as np
     cls = model.__class__
     cls.forward = magcache_eval_forward
     cls.magcache_thresh, cls.magcache_K = thresh, K
@@ -677,12 +599,7 @@ def teacache_forward(self, x, t, context, seq_len, clip_fea=None, y=None):
     _lib.check(_lib.lib.mc_tea_decide(ctypes.byref(cfg), ctypes.byref(st), dist, ctypes.byref(calc)))
     self.accumulated_rel_l1_distance_even, self.accumulated_rel_l1_distance_odd = st.accumulated[0], st.accumulated[1]
     setattr(self, "previous_e0_" + suffix, modulated.clone().view((e0 if self.use_ref_steps else e).shape))  # :549 / :564
-    cur = getattr(self, "previous_residual_" + suffix)
-    if cur is None:
-        eng.res_valid[slot] = False
-    elif torch.is_tensor(cur) and cur.data_ptr() != eng.res[slot].data_ptr():
-        eng.res[slot].copy_(cur.reshape(eng.res[slot].shape))
-        eng.res_valid[slot] = True
+    eng.res_valid[slot] = _adopt_residual(getattr(self, "previous_residual_" + suffix), eng.res[slot], eng.res_valid[slot])
     eng.hit_sum_bf16 = True  # `x += self.previous_residual_*` in place on the bf16 patch embedding (:569 / :577): the sum is rounded to bf16
     try:
         out = eng.forward("miss" if calc.value else "hit", slot)

@@ -70,7 +70,8 @@ def _f32(t, device):
 
 
 def _bias_autocast(t, device):
-    """Under bf16 autocast nn.Linear casts its bias to bf16 too; the epilogue adds it in fp32, so keep the rounded value as fp32."""
+    """Under bf16 autocast nn.Linear casts its bias to bf16 too; the epilogue adds it in fp32, so keep the rounded value as fp32.
+    The MMDiT engines keep their (bf16) biases and norm weights this way as well."""
     return t.detach().to(device=device, dtype=torch.bfloat16).float().contiguous()
 
 
@@ -356,10 +357,12 @@ class WanEngine:
         return self._rope[key]
 
     # ------------------------------------------------------------------------------------------ prologue (:229-275)
-    def stage_inputs(self, latent, t, context, clip_fea=None, y=None, vace_context=None, vace_scale=1.0, pad_row=0):
+    def stage_inputs(self, latent, t, context, clip_fea=None, y=None, vace_context=None, vace_scale=1.0, n_pad=0):
         """Copy one call's inputs into the engine's fixed buffers (outside any captured graph): latent fp32 [C, F, H, W],
         t tensor [1], context [L <= text_len, text_dim] (zero-padded to text_len, cast to bf16 as autocast would); i2v also
-        y [C_y, F, H, W] (concatenated under the latent channels, magcache_generate.py:233-234) and clip_fea [1, 257, clip_dim]."""
+        y [C_y, F, H, W] (concatenated under the latent channels, magcache_generate.py:233-234) and clip_fea [1, 257, clip_dim].
+        `n_pad` (calibration only): the zero rows the reference appends after the tokens (seq_len - token count); `calibrate` weights
+        one representative pad row by that count."""
         d = self.dims
         C, Fr, H, W = latent.shape
         if d.model_type == "i2v":
@@ -368,7 +371,8 @@ class WanEngine:
         if C + c_y != d.in_dim:
             raise ValueError(f"magcache_b200: {C}+{c_y} input channels, the patch embedding takes {d.in_dim}")
         self.grid = (Fr, H // 2, W // 2)
-        self._workspace(self.grid[0] * self.grid[1] * self.grid[2], pad_row)
+        self.n_pad = n_pad
+        self._workspace(self.grid[0] * self.grid[1] * self.grid[2], 1 if n_pad else 0)
         shape = (C + c_y, Fr, H, W)
         if self.s_lat is None or tuple(self.s_lat.shape) != shape:
             self.s_lat = torch.empty(shape, dtype=torch.float32, device=self.device)
@@ -475,21 +479,21 @@ class WanEngine:
         return self.x0, e, e0, self.ctx
 
     # ------------------------------------------------------------------------------------------ one patched forward
-    def _body(self, kind, slot):
+    def _body(self, kind, slot, step=None):
         """prologue -> {hit: head(x0 + residual) | miss: block stack, residual = x - x0, head(x)} on the staged inputs."""
         self._slot = slot
-        if self._native_ok():
+        if self._native_ok(step):
             return self._native_body(kind, slot)
         x0, e, e0, ctx = self.prologue(need_ctx=(kind != "hit"))
         if kind == "hit":
             # `x + residual_x` (:295) is formed inside the head kernel; TeaCache's in-place bf16 `x += residual` rounds the sum first
-            return self.head(x0, e, self.grid, residual=self.res[slot], round_sum_to_bf16=self.hit_sum_bf16)
+            return self.head(x0, e, self.grid, residual=self.res[slot], round_sum_to_bf16=self.hit_sum_bf16, step=step)
         xs = self.run_blocks(x0, e0, ctx, self.grid)
         ops.residual_sub(xs, x0, out=self.res[slot])  # magcache_generate.py:299, written into the slot's fixed buffer
-        return self.head(xs, e, self.grid)
+        return self.head(xs, e, self.grid, step=step)
 
-    def _native_ok(self):
-        if not self.native or self.shard is not None or self.runs is not None or self.pad_row or self._step is not None or self.hit_sum_bf16:
+    def _native_ok(self, step):
+        if not self.native or self.shard is not None or self.runs is not None or self.pad_row or step is not None or self.hit_sum_bf16:
             return False
         from . import native
         return native.supported(self.dims) and getattr(ops, "PROFILE", None) is None
@@ -511,7 +515,8 @@ class WanEngine:
         """Fold the caller loop's CFG combine + scheduler update (eval/.../wan_magcache.py:301-310) into the head pass of the NEXT
         forward, which must be the unconditional call of the step whose conditional prediction is `cond`: that forward then returns
         `coef_x * x_latent + coef_v * (uncond + guide_scale * (cond - uncond))` (written into `out`, which may be `x_latent` itself)
-        instead of the unconditional prediction. One-shot; bit-equal to the plain forward followed by `ops.cfg_step`."""
+        instead of the unconditional prediction. One-shot: the next `forward` or `calibrate` takes it off the engine, whether it
+        succeeds or not. Bit-equal to the plain forward followed by `ops.cfg_step`."""
         if self.shard is not None:
             raise NotImplementedError("magcache_b200: the fused step is built for the unsharded engine (sharded runs use ops.cfg_step)")
         if len(self.head_groups) != 1:
@@ -520,13 +525,11 @@ class WanEngine:
 
     def forward(self, kind, slot):
         """Run (or replay) one forward of the given kind for CFG slot `slot`; returns a fresh fp32 [C, F, H, W] tensor."""
+        step, self._step = self._step, None
         if kind == "hit" and not self.res_valid[slot]:
             raise TypeError("magcache_b200: cache hit with an empty residual_cache slot (reference: Tensor + NoneType)")
-        if not self.use_graphs or self._step is not None:  # an armed step carries per-step scalars: never captured
-            try:
-                out = self._body(kind, slot)
-            finally:
-                self._step = None
+        if not self.use_graphs or step is not None:  # an armed step carries per-step scalars: never captured
+            out = self._body(kind, slot, step)
         else:
             key = (kind, slot, self.hit_sum_bf16)
             st = self._graphs.get(key)
@@ -550,6 +553,33 @@ class WanEngine:
         if kind == "miss":
             self.res_valid[slot] = True
         return out
+
+    def calibrate(self, slot, prev):
+        """The calibration twin of `forward("miss", slot)` (MagCache4Wan2.1/magcache_generate.py:80-194): always runs the block stack.
+        `prev`: the previous fp32 residual of this CFG branch (N x D elements, any shape) or None. Returns (head output, residual,
+        (norm_ratio, norm_std, cos_dis) against `prev` or None). The residual is a new fp32 [N, D] tensor on every call: `prev` may
+        alias an earlier one, so nothing is written into the engine's residual slots."""
+        step, self._step = self._step, None
+        self._slot = slot
+        x0, e, e0, ctx = self.prologue()
+        xs = self.run_blocks(x0, e0, ctx, self.grid)
+        if prev is None:
+            residual, stats = ops.residual_sub(xs, x0), None
+        elif self.pad_row:
+            # seq_len > token count: rows [n_tok, seq_len) of the reference's tensors are identical copies of the one pad row computed
+            # here; its three per-row terms enter the means n_pad times (:167-169 average over dim 1 of [1, seq_len, D])
+            prev, n, wgt, keep = prev.view(x0.shape), self.n_keys, float(self.n_pad), {}
+            ops.residual_sub_stats(xs[n:], x0[n:], prev[n:].contiguous(), reduce=lambda st: keep.setdefault("pad", st.clone()))
+            residual_tok, stats = ops.residual_sub_stats(
+                xs[:n], x0[:n], prev[:n].contiguous(), reduce=lambda st: st + keep["pad"] * st.new_tensor([wgt, wgt, wgt, wgt]))
+            residual = torch.cat([residual_tok, xs[n:] - x0[n:].float()])
+        else:
+            reduce = None
+            if self.shard is not None:  # the statistics are sums over tokens: add the partial sums of every token shard
+                from .shard import allreduce_stats
+                reduce = lambda st: allreduce_stats(st, self.shard.group)  # noqa: E731
+            residual, stats = ops.residual_sub_stats(xs, x0, prev.view(x0.shape), reduce=reduce)
+        return self.head(xs, e, self.grid, step=step), residual, stats
 
     # ------------------------------------------------------------------------------------------ block stack (:297-298)
     def run_blocks(self, x0, e0, ctx, grid):
@@ -664,7 +694,9 @@ class WanEngine:
             ops.gemm(a[r0:r1], w, bias, E.MC_EPI_BIAS_GATE_RESID, out=xs[r0:r1], gate=self.em[u][gate_idx], tag=tag)
 
     # ------------------------------------------------------------------------------------------ epilogue (:304-305)
-    def head(self, x, e, grid, residual=None, round_sum_to_bf16=False):
+    def head(self, x, e, grid, residual=None, round_sum_to_bf16=False, step=None):
+        """head + unpatchify of the stream `x` (or of x0 + `residual` on a hit). `step`: the `arm_step` tuple of the forward in flight,
+        applied in the epilogue."""
         w, G = self.w, len(self.head_groups)
         tag = "head_hit_fused" if residual is not None else "head"
         kw = dict(c_out=16, eps=self.dims.eps, tag=tag, round_sum_to_bf16=round_sum_to_bf16)
@@ -680,14 +712,14 @@ class WanEngine:
             row_offset = self.shard.start
         if self.runs is None and G == 1:  # one timestep, 16 output channels: a single launch
             (wt, hb), = self.head_groups
-            if self.shard is None and self._step is not None:
-                kw["step"], out = self._step[:5], self._step[5]
+            if self.shard is None and step is not None:
+                kw["step"], out = step[:5], step[5]
             out = ops.head_unpatchify(x, w.head_mod, e, wt, hb, grid, residual=residual, row_offset=row_offset, out=out, peer_outs=peer_outs,
                                       prep=self._head_prep[(0, 0)], **kw)
         else:
             # per-token timesteps and / or more than 16 output channels: one launch per (row range, channel group), each writing
             # its own rows x channels of the same output tensor
-            if self._step is not None:
+            if step is not None:
                 raise NotImplementedError("magcache_b200: the fused step is built for one timestep and 16 output channels (use ops.cfg_step)")
             n_rows = x.shape[0]
             if out is None:

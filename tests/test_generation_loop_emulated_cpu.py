@@ -98,6 +98,32 @@ def test_fused_step_equals_two_calls_plus_cfg_step(emulated):
     assert b_model._mc_engine._step is None
 
 
+def test_fused_step_under_calibration(emulated):
+    """A calibration-installed model (`init_magcache_calibration`, magcache_generate.py:921-928) driven by `FlowEulerSampler.denoise`:
+    the armed step is applied once, by the unconditional call's head, and never survives into the next step's conditional call —
+    latents bit-equal to the two calls followed by `sampler.step`, same statistics."""
+    steps, guide = 4, 5.0
+    a_model, b_model = (_models(lambda c: None, lambda m: mc.init_magcache_calibration(m, steps))[1] for _ in range(2))
+    for m in (a_model, b_model):
+        type(m).calibration_dir = None
+    g = torch.Generator().manual_seed(2)
+    lat = torch.randn(16, 2, 8, 8, generator=g)
+    ctx, ctx_null = torch.randn(9, 128, generator=g), torch.randn(7, 128, generator=g)
+    sig = mc.sampling_sigmas(steps, 5.0)
+    sa, sb = mc.FlowEulerSampler(sig), mc.FlowEulerSampler(sig)
+    xa, xb = lat.clone(), lat.clone()
+    with torch.no_grad():
+        for i in range(steps):
+            t = torch.tensor([sa.timestep], dtype=torch.float32)
+            cond = a_model([xa], t=t, context=[ctx], seq_len=32)[0]
+            uncond = a_model([xa], t=t, context=[ctx_null], seq_len=32)[0]
+            xa = sa.step(cond, uncond, guide, xa)
+            sb.denoise(b_model, xb, t, ctx, ctx_null, 32, guide)
+            assert b_model._mc_engine._step is None, i
+            assert torch.equal(xa, xb), i
+    assert len(b_model.norm_ratio) == 2 * steps - 2 and b_model.norm_ratio == a_model.norm_ratio
+
+
 def test_teacache_generation_loop(emulated):
     steps, coef = 8, [0.02, 0.04, 0.0]
     ref, ours = _models(lambda c: wan_ref.install_teacache(c, steps, 0.08, coef), lambda m: mc.init_teacache(m, steps, teacache_thresh=0.08, coefficients=coef))

@@ -67,7 +67,7 @@ def _worker(rank, world, initfile, results, family):
         res_err = float((loc_res.float() - full_res[eng.shard.start:eng.shard.stop].float()).abs().max() / full_res.float().abs().max())
         # calibration twin (magcache_flux.py:21-231 / magcache_sample_video.py:163-290) on the sharded engine: the three statistics are
         # sums over the image tokens, so the ranks' partial sums are added before they are finalised — same lists as one engine
-        cal = {}
+        cal, cal_shard = {}, {}
         for name in ("single", "sharded"):
             m = copy.deepcopy(model)
             m.__class__ = type("C_" + name, (m.__class__,), {})
@@ -79,7 +79,8 @@ def _worker(rank, world, initfile, results, family):
                 for i in range(4):
                     call(m, i)
             cal[name] = [list(getattr(m, k)) for k in ("norm_ratio", "norm_std", "cos_dis")]
-        results[rank] = (errs, res_err, eng.n_img, eng.n_img_total, eng.S_keys, cal)
+            cal_shard[name] = getattr(m, eng_attr).shard is not None
+        results[rank] = (errs, res_err, eng.n_img, eng.n_img_total, eng.S_keys, cal, cal_shard)
     finally:
         dist.destroy_process_group()
 
@@ -92,7 +93,8 @@ def test_sharded_mmdit_engine_equals_single_world2(family):
         mp.spawn(_worker, args=(2, os.path.join(d, "init"), results, family), nprocs=2, join=True)
         assert set(results.keys()) == {0, 1}
         for r in (0, 1):
-            errs, res_err, n_loc, n_tot, s_keys, cal = results[r]
+            errs, res_err, n_loc, n_tot, s_keys, cal, cal_shard = results[r]
+            assert cal_shard == {"single": False, "sharded": True}  # enable_token_shard reaches the calibration engine too
             assert all(len(v) == 3 for v in cal["single"]) and all(len(v) == 3 for v in cal["sharded"]), cal
             for a, b in zip(sum(cal["sharded"], []), sum(cal["single"], [])):
                 assert abs(a - b) <= 2e-2 * abs(b) + 2e-3, cal
